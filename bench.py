@@ -227,6 +227,16 @@ def parity_block(gk, gd, rk, rd, rtol=1e-5, atol=1e-6):
             "max_rel_dist_err": float(rel.max()) if rel.size else 0.0}
 
 
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs DIR: what the timed path returned to its caller in the last timed step, one DIR/<name>.npy per array,
+    distances as float32 and keys / counts as float64 (exact: keys stay far below 2**53).  The inputs depend only on the
+    arguments (seeded generators), so two builds of the project can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+
+
 def peaks():
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
@@ -279,6 +289,9 @@ def run_reference(args, wl):
         t0 = time.perf_counter()
         keys, dists, counts, comp, vis = idx.search_batch(q, wl["k"], threads=cores)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:  # per_step follows the measured rate: the first min(B, 64) queries of the step are always in it
+        m = min(B, 64)
+        dump_outputs(args.dump_outputs, keys=keys[:m], distances=dists[:m], counts=counts[:m])
     total = sum(times)
     value = args.steps * per_step / total
     sample = ("reference builds its own graph over the first %d rows of the %d-row corpus generator (%.0f s, %d threads); each step = "
@@ -314,9 +327,11 @@ def run_reference_port(args, wl):
     times = []
     for s in range(args.steps + args.warmup):
         t0 = time.perf_counter()
-        idx.search_batch(Q[s * per_step:(s + 1) * per_step], wl["k"])
+        keys, dists, counts, _ = idx.search_batch(Q[s * per_step:(s + 1) * per_step], wl["k"])
         if s >= args.warmup:
             times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, keys=keys, distances=dists, counts=counts)
     value = args.steps * per_step / sum(times)
     sample = "oracle PORT (oracle/_ref missing): 1 thread, own graph over the first %d rows (%.0f s), %d queries per step" % (
         n_ref, t_build, per_step)
@@ -605,6 +620,11 @@ def run_ours(args, wl):
     barrier()
     ms = ev[0].elapsed_time(ev[1])
     launches = api.kernel_launches() - launches0
+    if args.dump_outputs and rank == 0:  # the last timed step's results, before anything else reuses the buffers
+        if world > 1:
+            dump_outputs(args.dump_outputs, keys=m_keys, distances=m_dists)
+        else:
+            dump_outputs(args.dump_outputs, keys=out_keys, distances=out_dists, counts=out_counts)
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -980,6 +1000,8 @@ def run_group(args, wl):
         step_device(s)
     ev[1].record(stream)
     barrier()
+    if args.dump_outputs and rank == 0:  # the last timed step's results, before anything else reuses the buffers
+        dump_outputs(args.dump_outputs, keys=out_keys, distances=out_dists, counts=out_counts)
     t = torch.tensor([ev[0].elapsed_time(ev[1])], dtype=torch.float64, device=dev)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
@@ -1102,7 +1124,11 @@ def main():
     ap.add_argument("--ref-rows", type=int, default=200_000,
                     help="--impl reference: corpus prefix the reference indexes (fixed, so the arm is the same on every box and N)")
     ap.add_argument("--per-step-stats", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last timed step (keys, distances, counts) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl)

@@ -1,10 +1,13 @@
 """TEST INFRASTRUCTURE: a stand-in for `lantern_b200.api` that answers through the CPU oracle (oracle/portlib.py).
 
-Only tests/test_bench_dryrun.py uses it, to walk bench.py's `run_ours` glue (argument plumbing, the JSON line, the
+tests/test_bench_dryrun.py uses it to walk bench.py's `run_ours` glue (argument plumbing, the JSON line, the
 cpu_baseline / parity / sharding branches) on a machine without a GPU.  It mirrors the few entry points bench.py calls,
-with the same signatures (raw pointers in, results written through raw pointers).  Nothing here is a product path."""
+with the same signatures (raw pointers in, results written through raw pointers).  The oracle also stands in for the
+compiled reference (`oracle.reflib`) that cpu_baseline and the `--impl reference` arm (tests/test_bench_contract.py) drive,
+so that neither walk needs a reference build.  Nothing here is a product path."""
 import ctypes as C
 import time
+import types
 
 import numpy as np
 
@@ -44,12 +47,15 @@ def install(bench, setattr_=setattr, setitem=None):
     import torch
 
     import lantern_b200
+    import oracle.reflib
     if setitem is None:
         def setitem(d, k, v):
             d[k] = v
     me = sys.modules[__name__]
     setitem(sys.modules, "lantern_b200.api", me)
     setattr_(lantern_b200, "api", me)
+    setitem(sys.modules, "oracle.reflib", REFLIB)
+    setattr_(oracle, "reflib", REFLIB)
     setattr_(torch.cuda, "set_device", lambda d: None)
     setattr_(torch.cuda, "synchronize", lambda *a: None)
     setattr_(torch.cuda, "current_stream", lambda *a: HostStream())
@@ -160,3 +166,31 @@ def merge_shards_device(d_keys, d_dists, shards, nq, k, d_out_keys, d_out_dists,
     view(d_out_keys, (nq, k), np.uint64)[:] = np.take_along_axis(keys, order, 1)
     view(d_out_dists, (nq, k), np.float32)[:] = np.take_along_axis(dists, order, 1)
     LAUNCHES[0] += 1
+
+
+class RefIndex:
+    """The reference's index as bench.py drives it: build over rows (--impl reference) or load the engine's index file
+    (cpu_baseline), then search query batches."""
+
+    def __init__(self, dim, metric="l2sq", quant="f32", M=16, efc=128, ef=64, threads=1):
+        self.p = portlib.PortIndex(dim, metric, quant, M=M, efc=efc, ef=ef)
+
+    def reserve(self, n):
+        self.p.reserve(n)
+
+    def add_batch(self, keys, vecs, threads=None):
+        for key, row in zip(keys, vecs):
+            self.p.add(int(key), row)
+
+    def load_buffer(self, buf):
+        buf = np.ascontiguousarray(buf, dtype=np.uint8)
+        self.p.reserve(int(buf[80:88].view(np.uint64)[0]))  # node count of the file header
+        self.p.load_buffer(buf)
+
+    def search_batch(self, queries, k, threads=None):
+        keys, dists, counts, tot = self.p.search_batch(queries, k)
+        return keys, dists, counts, tot["computed_distances"], tot["visited_members"]
+
+
+REFLIB = types.SimpleNamespace(available=lambda: True, lib=lambda: types.SimpleNamespace(refx_hardware_threads=lambda: 1),
+                               RefIndex=RefIndex)

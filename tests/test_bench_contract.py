@@ -1,18 +1,22 @@
 """bench.py contract checks that need no GPU: the reference arm runs on the host cores and prints one JSON line with the
-keys the driver reads; the workload table is self-consistent."""
+keys a reader of the benchmark relies on; the workload table is self-consistent."""
 import json
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_reference_arm_prints_contract_line(ref):
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "cfg2s", "--steps", "2",
-                          "--warmup", "3", "--ref-rows", "3000", "--ref-seconds", "1"], capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stderr[-2000:]
-    line = json.loads(out.stdout.strip().splitlines()[-1])
+def test_reference_arm_prints_contract_line(monkeypatch, capsys):
+    """The arm's glue, with the oracle standing in for the compiled reference (tests/fake_engine.py)."""
+    sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
+    import bench
+    import fake_engine
+    fake_engine.install(bench, monkeypatch.setattr, monkeypatch.setitem)
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--workload", "cfg2s", "--steps", "2", "--warmup", "3",
+                                      "--ref-rows", "3000", "--ref-seconds", "1"])
+    bench.main()
+    line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "queries/s" and line["higher_is_better"] is True
     for key in ("metric", "value", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "vs_baseline", "dtype", "data", "config",
                 "cpu_baseline", "e2e"):

@@ -1,7 +1,8 @@
 """bench.py's own arm walked end to end on the CPU: the engine is replaced by tests/fake_engine.py (the oracle behind the
 same entry points) and torch.cuda's stream/event calls by host stand-ins, so that every line of the N=1 glue -- data
-generation, build calls, timed loops, roofline block, e2e loop, cpu_baseline over the reference (oracle/_ref), parity
-block, the JSON line -- executes here before it is trusted on a GPU box.  No number printed by this test means anything."""
+generation, build calls, timed loops, roofline block, e2e loop, cpu_baseline over the reference (the oracle stands in for
+it as well), parity block, the JSON line -- executes here before it is trusted on a GPU box.  No number printed by this test
+means anything."""
 import json
 import os
 import sys
@@ -15,7 +16,7 @@ CONTRACT_KEYS = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per
 
 
 @pytest.fixture
-def host_bench(monkeypatch, ref):
+def host_bench(monkeypatch):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import bench
@@ -75,7 +76,7 @@ def test_default_workload_is_the_one_the_metric_names(host_bench):
 
 
 @pytest.mark.parametrize("big", [False, True])
-def test_two_rank_glue_over_gloo(ref, big):
+def test_two_rank_glue_over_gloo(big):
     """The sharded path (row-range shards, all-gather of per-shard top-k, merge, recall-matched per-shard ef, max-over-ranks
     timing) on two CPU ranks over gloo; `big` = the branch the 10M-row default takes (recorded 1-GPU recall as the target)."""
     env = dict(os.environ, DRYRUN_BIG="1" if big else "", MASTER_ADDR="127.0.0.1")
@@ -95,3 +96,25 @@ def test_two_rank_glue_over_gloo(ref, big):
     assert ("recorded" in sh["recall_target_source"]) == big
     assert ("replicated_comparison" in sh) == (not big)
     assert line["e2e"]["h2d_bytes_per_step"] == 2 * 8 * 32 * 4 and line["value"] > 0 and 0.5 < line["recall_at_10"] <= 1.0
+
+
+def test_dump_outputs_are_the_last_timed_step(host_bench, monkeypatch, capsys, tmp_path):
+    """--dump-outputs: the arrays the timed path returned in its last step, as float npy files, identical across runs with the
+    same arguments."""
+    import numpy as np
+    dumps = []
+    for run_dir in ("a", "b"):
+        line, err = run(host_bench, monkeypatch, capsys, "--workload", "tiny", "--steps", "5", "--warmup", "3", "--no-cpu-baseline",
+                        "--dump-outputs", str(tmp_path / run_dir))
+        assert line["steps"] == 5
+        dumps.append({n: np.load(tmp_path / run_dir / (n + ".npy")) for n in ("keys", "distances", "counts")})
+    a, b = dumps
+    assert a["keys"].shape == a["distances"].shape == (8, 10) and a["counts"].shape == (8,)
+    assert a["keys"].dtype == np.float64 and a["distances"].dtype == np.float32 and a["counts"].dtype == np.float64
+    assert all(np.array_equal(a[n], b[n]) for n in a)
+    # step s searches query batch s % pool: the last timed step (s = 7, pool 8) is the last batch of the query pool
+    bench = host_bench
+    X = bench.structured_torch(3000, 32, bench.SEED_CORPUS, "cpu").numpy()
+    Q = bench.structured_torch(8 * 8, 32, bench.SEED_QUERY, "cpu").numpy()[7 * 8:]
+    d = ((Q[:, None, :] - X[a["keys"].astype(np.int64) - 1]) ** 2).sum(-1)
+    assert np.allclose(d, a["distances"], rtol=1e-4, atol=1e-4)

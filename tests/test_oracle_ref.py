@@ -1,94 +1,94 @@
-"""The plain-C restatement against the compiled reference itself (skipped where oracle/_ref is absent)."""
-import struct
+"""The plain-C restatement against the compiled reference itself.
+
+tests/golden/oracle_ref_v1.npz holds what the UNMODIFIED reference (oracle/_ref) answered for exactly these inputs; it is
+written by tests/golden/make_oracle_ref.py, and test_golden.py checks that it still reproduces from oracle/_ref wherever
+that is built.  Index files are compared through their SHA-256 digests."""
+import hashlib
+import os
+import sys
 
 import numpy as np
 import pytest
 
+sys.path.insert(0, os.path.dirname(__file__))
+from util import scalar_kind_inputs, with_vectors  # noqa: E402
 
-def trim(buf, stored_bytes=None):
-    """The reference's save_buffer may leave slack after the last node; pq nodes carry `num_subvectors` code bytes instead
-    of the header's vector_size_bytes."""
-    n, M, M0 = struct.unpack_from("<QQQ", buf, 80)
-    vsz, = struct.unpack_from("<Q", buf, 120)
-    if stored_bytes is not None:
-        vsz = stored_bytes
-    off, b = 136, bytes(buf)
-    for _ in range(n):
-        lvl, = struct.unpack_from("<h", b, off + 8)
-        off += 10 + 4 + 6 * M0 + lvl * (4 + 6 * M) + vsz
-    return np.array(buf[:off])
+G = np.load(os.path.join(os.path.dirname(__file__), "golden", "oracle_ref_v1.npz"))
+METRICS = ("l2sq", "cos")
+VARIANTS = ("f16", "i8", "b1", "pq")
+NO_KEY = np.iinfo(np.uint64).max
+
+
+def same_file(buf, want_sha256):
+    return hashlib.sha256(bytes(buf)).digest() == bytes(want_sha256)
+
+
+def searches(idx, Q, ks, width):
+    """One query at a time; row i holds the ks[i] results, padded to `width` with NO_KEY / +inf (the fixture's layout)."""
+    keys = np.full((len(Q), width), NO_KEY, np.uint64)
+    dists = np.full((len(Q), width), np.inf, np.float32)
+    for i, (q, k) in enumerate(zip(Q, ks)):
+        kk, dd, _ = idx.search(q, k)
+        keys[i, :len(kk)], dists[i, :len(kk)] = kk, dd
+    return keys, dists
 
 
 @pytest.mark.parametrize("n,d,M,efc,ef,metric", [(1500, 32, 16, 128, 64, "l2sq"), (2000, 24, 6, 40, 20, "l2sq"), (1200, 48, 16, 96, 50, "cos")])
-def test_build_and_search_byte_exact_on_integer_data(port, ref, n, d, M, efc, ef, metric):
+def test_build_and_search_byte_exact_on_integer_data(port, n, d, M, efc, ef, metric):
     rng = np.random.default_rng(n)
     X = rng.integers(-8, 9, (n, d)).astype(np.float32)
     Q = rng.integers(-8, 9, (150, d)).astype(np.float32)
-    r = ref.RefIndex(d, metric, M=M, efc=efc, ef=ef)
     p = port.PortIndex(d, metric, M=M, efc=efc, ef=ef)
-    r.reserve(n), p.reserve(n)
+    p.reserve(n)
     for i in range(n):
-        r.add(i + 1, X[i]), p.add(i + 1, X[i])
-    assert np.array_equal(trim(r.save_buffer()), p.save_buffer())
-    for q in Q:
-        rk, rd = r.search(q, 10)
-        pk, pd, st = p.search(q, 10)
-        assert np.array_equal(rk, pk) and np.array_equal(rd, pd)
+        p.add(i + 1, X[i])
+    name = "int_%s_n%d" % (metric, n)
+    assert same_file(p.save_buffer(), G[name + "_file_sha256"])
+    pk, pd = searches(p, Q, [10] * len(Q), 10)
+    assert np.array_equal(G[name + "_keys"], pk) and np.array_equal(G[name + "_dists"], pd)
 
 
-def test_counters_match_reference(port, ref):
+def test_counters_match_reference(port):
     """computed_distances / visited_members (index.hpp:2726-2727) -- the quantity the roofline's algorithmic bytes use."""
-    import ctypes as C
     rng = np.random.default_rng(5)
     X = rng.integers(-8, 9, (2000, 32)).astype(np.float32)
-    r = ref.RefIndex(32, "l2sq", M=16, efc=128, ef=64)
     p = port.PortIndex(32, "l2sq", M=16, efc=128, ef=64)
-    r.reserve(2000), p.reserve(2000)
+    p.reserve(2000)
     for i in range(2000):
-        r.add(i + 1, X[i]), p.add(i + 1, X[i])
-    L = ref.lib()
-    for q in rng.integers(-8, 9, (50, 32)).astype(np.float32):
-        keys, dists = np.zeros(10, np.uint64), np.zeros(10, np.float32)
-        comp, vis = C.c_uint64(), C.c_uint64()
-        L.refx_search_stats(r.h, q.ctypes.data, 10, keys.ctypes.data, dists.ctypes.data, C.byref(comp), C.byref(vis))
+        p.add(i + 1, X[i])
+    Q = rng.integers(-8, 9, (50, 32)).astype(np.float32)
+    for q, comp, vis in zip(Q, G["counters_computed_distances"], G["counters_visited_members"]):
         pk, pd, st = p.search(q, 10)
-        assert st.computed_distances == comp.value and st.visited_members == vis.value
+        assert st.computed_distances == comp and st.visited_members == vis
 
 
-def test_float_data_ids_and_tolerance(port, ref):
+def test_float_data_ids_and_tolerance(port):
     rng = np.random.default_rng(11)
     X = rng.standard_normal((1500, 64)).astype(np.float32)
-    r = ref.RefIndex(64, "cos", M=16, efc=128, ef=64)
-    r.reserve(1500)
-    for i in range(1500):
-        r.add(i + 1, X[i])
     p = port.PortIndex(64, "cos", M=16, efc=128, ef=64)
     p.reserve(1500)
-    p.load_buffer(trim(r.save_buffer()))  # same graph, the reference's own bytes
+    p.load_buffer(with_vectors(G["float_cos_graph"], X))  # same graph, the reference's own bytes
     same = 0
-    for q in rng.standard_normal((200, 64)).astype(np.float32):
-        rk, rd = r.search(q, 10)
+    for q, rk, rd in zip(rng.standard_normal((200, 64)).astype(np.float32), G["float_cos_keys"], G["float_cos_dists"]):
         pk, pd, _ = p.search(q, 10)
         assert np.allclose(rd, pd, rtol=1e-5, atol=1e-6)
         same += np.array_equal(rk, pk)
     assert same >= 198
 
 
-def test_pq_128_centroid_quirk(port, ref):
+def test_pq_128_centroid_quirk(port):
     """codebook_t::compress never picks centroids >= 128 (signed char loop, lantern_storage.hpp:123)."""
     rng = np.random.default_rng(2)
     d, nsub, ncent = 16, 4, 256
     cb = rng.standard_normal((ncent, d)).astype(np.float32)
     X = rng.standard_normal((300, d)).astype(np.float32)
-    r = ref.RefIndex(d, "l2sq", M=8, efc=32, ef=300, pq=True, num_centroids=ncent, num_subvectors=nsub, codebook=cb)
-    r.reserve(300)
-    for i in range(300):
-        r.add(i + 1, X[i])
     codes = port.pq_compress(cb, X, nsub, compat128=True)
     assert codes.max() < 128
     dec = port.pq_decompress(cb, codes)
     q = rng.standard_normal(d).astype(np.float32)
-    rk, rd = r.search(q, 300)  # ef = N -> (almost) every node, distances = raw query vs decoded candidate
+    # the reference's pq index over X with ef = N answers (almost) every node for q; its distances are raw query vs decoded
+    # candidate
+    rk, rd = G["pq256_keys"], G["pq256_dists"]
     mine = ((dec[rk.astype(int) - 1] - q) ** 2).sum(1)
     assert np.allclose(mine, rd, rtol=1e-5, atol=1e-6)
     full = port.pq_compress(cb, X, nsub, compat128=False)
@@ -117,71 +117,38 @@ def test_engine_tie_order_mode_equals_reference_without_ties(port):
     assert np.mean(d1 == d2) > 0.97
 
 
-def test_property_port_equals_reference_on_random_small_configs(port, ref):
-    """Property test (hypothesis): for random (N, d, M, ef_construction, ef, metric) and integer-valued data the
-    restatement and the compiled reference write the same index file and return the same ids and distances."""
-    from hypothesis import given, settings, strategies as st
-
-    @settings(max_examples=20, deadline=None)
-    @given(n=st.integers(2, 300), d=st.integers(1, 20), M=st.sampled_from([2, 3, 4, 8, 16]), efc=st.integers(4, 64),
-           ef=st.integers(1, 48), metric=st.sampled_from(["l2sq", "cos"]), seed=st.integers(0, 10_000))
-    def check(n, d, M, efc, ef, metric, seed):
+def test_property_port_equals_reference_on_random_small_configs(port):
+    """Property test over the 28 seeded configurations (N, d, M, ef_construction, ef, metric) of the fixture -- the smallest
+    and largest of the ranges, then random draws: on integer-valued data the restatement writes the reference's index
+    file and returns its ids and distances."""
+    for cfg, want_file, want_k, want_d in zip(G["prop_configs"], G["prop_file_sha256"], G["prop_keys"], G["prop_dists"]):
+        n, d, M, efc, ef, metric, seed = (int(v) for v in cfg)
         rng = np.random.default_rng(seed)
         X = rng.integers(-5, 6, (n, d)).astype(np.float32)
-        r = ref.RefIndex(d, metric, M=M, efc=efc, ef=ef)
-        p = port.PortIndex(d, metric, M=M, efc=efc, ef=ef)
-        r.reserve(n), p.reserve(n)
+        p = port.PortIndex(d, METRICS[metric], M=M, efc=efc, ef=ef)
+        p.reserve(n)
         for i in range(n):
-            r.add(i + 1, X[i]), p.add(i + 1, X[i])
-        assert np.array_equal(trim(r.save_buffer()), p.save_buffer())
-        for q in rng.integers(-5, 6, (10, d)).astype(np.float32):
-            k = int(rng.integers(1, 12))
-            rk, rd = r.search(q, k)
-            pk, pd, _ = p.search(q, k)
-            assert np.array_equal(rk, pk) and np.array_equal(rd, pd)
-
-    check()
+            p.add(i + 1, X[i])
+        assert same_file(p.save_buffer(), want_file), cfg
+        Q = rng.integers(-5, 6, (10, d)).astype(np.float32)
+        pk, pd = searches(p, Q, [int(rng.integers(1, 12)) for _ in Q], want_k.shape[1])
+        assert np.array_equal(want_k, pk) and np.array_equal(want_d, pd), cfg
 
 
-def test_property_scalar_kinds_bits_and_pq(port, ref):
-    """Same property for the storage variants: f16 / i8 scalar quantisation (f32 in, cast on add), packed bits with the
-    hamming metric, and pq storage with a random codebook (stored side decoded, value side raw)."""
-    from hypothesis import given, settings, strategies as st
-
-    @settings(max_examples=20, deadline=None)
-    @given(n=st.integers(2, 200), sub=st.integers(1, 6), M=st.sampled_from([2, 4, 8]), efc=st.integers(4, 48),
-           ef=st.integers(1, 32), variant=st.sampled_from(["f16", "i8", "b1", "pq"]), metric=st.sampled_from(["l2sq", "cos"]),
-           seed=st.integers(0, 10_000))
-    def check(n, sub, M, efc, ef, variant, metric, seed):
-        rng = np.random.default_rng(seed)
-        kw, quant, d = {}, "f32", 4 * sub
-        if variant == "b1":
-            metric, quant, d = "hamming", "b1", 32 * sub
-            X = rng.integers(0, 256, (n, d // 8), dtype=np.uint8)
-            Q = rng.integers(0, 256, (8, d // 8), dtype=np.uint8)
-        else:
-            # small multiples of 1/4: exact in f16, and |x| * 100 stays an integer below the i8 clamp for the small ones
-            X = (rng.integers(-4, 5, (n, d)) / 4.0).astype(np.float32)
-            Q = (rng.integers(-4, 5, (8, d)) / 4.0).astype(np.float32)
-            if variant == "pq":
-                ncent = int(rng.integers(2, 9))
-                kw = dict(pq=True, num_centroids=ncent, num_subvectors=sub,
-                          codebook=(rng.integers(-4, 5, (ncent, d)) / 4.0).astype(np.float32))
-            else:
-                quant = variant
-        r = ref.RefIndex(d, metric, quant, M=M, efc=efc, ef=ef, **kw)
+def test_property_scalar_kinds_bits_and_pq(port):
+    """Same property for the storage variants (tests/util.py::scalar_kind_inputs), three seeded configurations for every
+    (variant, metric) pair: f16 / i8 scalar quantisation (f32 in, cast on add), packed bits with the hamming metric, and
+    pq storage with a random codebook (stored side decoded, value side raw)."""
+    for cfg, want_file, want_k, want_d in zip(G["kinds_configs"], G["kinds_file_sha256"], G["kinds_keys"], G["kinds_dists"]):
+        n, sub, M, efc, ef, variant, metric, seed = (int(v) for v in cfg)
+        rng, X, Q, d, metric, quant, kw = scalar_kind_inputs(n, sub, VARIANTS[variant], METRICS[metric], seed)
         p = port.PortIndex(d, metric, quant, M=M, efc=efc, ef=ef, **kw)
-        r.reserve(n), p.reserve(n)
+        p.reserve(n)
         for i in range(n):
-            r.add(i + 1, X[i]), p.add(i + 1, X[i])
-        assert np.array_equal(trim(r.save_buffer(), sub if variant == "pq" else None), p.save_buffer())
-        for q in Q:
-            k = int(rng.integers(1, 10))
-            rk, rd = r.search(q, k)
-            pk, pd, _ = p.search(q, k)
-            assert np.array_equal(rk, pk) and np.array_equal(rd, pd)
-
-    check()
+            p.add(i + 1, X[i])
+        assert same_file(p.save_buffer(), want_file), cfg
+        pk, pd = searches(p, Q, [int(rng.integers(1, 10)) for _ in Q], want_k.shape[1])
+        assert np.array_equal(want_k, pk) and np.array_equal(want_d, pd), cfg
 
 
 @pytest.mark.parametrize("metric,quant", [("l2sq", "f32"), ("cos", "f32"), ("hamming", "b1")])
@@ -239,20 +206,19 @@ def test_batched_build_model_is_deterministic_and_as_good_as_sequential(port):
 
 
 @pytest.mark.parametrize("metric,scale", [("l2sq", 3.0), ("l2sq", 8.0), ("cos", 3.0)])
-def test_kmeans_restatement_equals_the_reference(ref, port, metric, scale):
+def test_kmeans_restatement_equals_the_reference(port, metric, scale):
     """PQ codebook training: the UNMODIFIED reference k-means (lantern_hnsw/src/hnsw/product_quantization.c compiled against
     the stand-in postgres.h of oracle/pg_shim/, PRNG scripted so that both sides start from the same rows) against the
     plain-C restatement ora_kmeans -- bit for bit, for 1, 3 and up to 25 Lloyd rounds, which pins row (f4) of SURVEY 8."""
-    if not ref.pq_available():
-        pytest.skip("oracle/_ref/liboracle_refpq.so not built")
     rng = np.random.default_rng(6)
     n, d, nsub, ncent = 3000, 24, 4, 16
     centers = rng.standard_normal((ncent, d)).astype(np.float32) * scale
     X = (centers[rng.integers(0, ncent, n)] + rng.standard_normal((n, d))).astype(np.float32)
     init = np.stack([rng.choice(n, ncent, replace=False) for _ in range(nsub)]).astype(np.uint32)
     seen_rounds = set()
+    name = "kmeans_%s_%g" % (metric, scale)
     for it in (1, 3, 25):
-        rcb = ref.ref_kmeans(X, nsub, ncent, init, metric, it)
+        rcb = G["%s_it%d" % (name, it)]
         pcb, rounds = port.kmeans(X, nsub, ncent, init, metric, it)
         assert np.array_equal(rcb.view(np.uint32), pcb.view(np.uint32)), np.abs(rcb - pcb).max()
         seen_rounds.add(rounds)
@@ -261,4 +227,4 @@ def test_kmeans_restatement_equals_the_reference(ref, port, metric, scale):
     # the hnsw_pq_index.sql fixture geometry: k == n, every init is a permutation, one round moves nothing
     Xc = np.repeat((np.arange(10) * 0.1).astype(np.float32)[:, None], 16, axis=1)
     perm = np.stack([rng.permutation(10) for _ in range(4)]).astype(np.uint32)
-    assert np.array_equal(ref.ref_kmeans(Xc, 4, 10, perm, "l2sq", 20), port.kmeans(Xc, 4, 10, perm, "l2sq", 20)[0])
+    assert np.array_equal(G[name + "_fixture"], port.kmeans(Xc, 4, 10, perm, "l2sq", 20)[0])

@@ -88,3 +88,43 @@ def graph_agreement(buf_a, buf_b, M, stored_bytes):
     assert la.keys() == lb.keys()
     same = sum(1 for k in la if la[k] == lb[k])
     return same / max(1, len(la))
+
+
+def with_vectors(graph, X):
+    """An index file from its vector-free form (tests/golden/make_oracle_ref.py::graph_only) and the rows in slot order."""
+    g = np.asarray(graph, dtype=np.uint8).tobytes()
+    n, M, M0 = (int(v) for v in np.frombuffer(g, np.uint64, 3, 80))
+    vsz = int(np.frombuffer(g, np.uint64, 1, 120)[0])
+    X = np.ascontiguousarray(X)
+    assert len(X) == n and X[0].nbytes == vsz, (len(X), n, X[0].nbytes, vsz)
+    out, off = [g[:136]], 136
+    for i in range(n):
+        lvl = int(np.frombuffer(g, np.int16, 1, off + 8)[0])
+        size = 10 + 4 + 6 * M0 + lvl * (4 + 6 * M)
+        out += [g[off:off + size], X[i].tobytes()]
+        off += size
+    assert off == len(g), (off, len(g))
+    return np.frombuffer(b"".join(out), np.uint8)
+
+
+def scalar_kind_inputs(n, sub, variant, metric, seed):
+    """Inputs of one configuration of tests/test_oracle_ref.py::test_property_scalar_kinds_bits_and_pq: f16 / i8 scalar
+    quantisation (f32 in, cast on add), packed bits with the hamming metric, or pq storage with a random codebook.  Small
+    multiples of 1/4: exact in f16, and |x| * 100 stays an integer below the i8 clamp for the small ones.  Returns the rng
+    (the test draws each query's k from it next), rows, queries, dimensions, metric, scalar kind and the pq arguments."""
+    rng = np.random.default_rng(seed)
+    kw, quant, d = {}, "f32", 4 * sub
+    if variant == "b1":
+        metric, quant, d = "hamming", "b1", 32 * sub
+        X = rng.integers(0, 256, (n, d // 8), dtype=np.uint8)
+        Q = rng.integers(0, 256, (8, d // 8), dtype=np.uint8)
+    else:
+        X = (rng.integers(-4, 5, (n, d)) / 4.0).astype(np.float32)
+        Q = (rng.integers(-4, 5, (8, d)) / 4.0).astype(np.float32)
+        if variant == "pq":
+            ncent = int(rng.integers(2, 9))
+            kw = dict(pq=True, num_centroids=ncent, num_subvectors=sub,
+                      codebook=(rng.integers(-4, 5, (ncent, d)) / 4.0).astype(np.float32))
+        else:
+            quant = variant
+    return rng, X, Q, d, metric, quant, kw
